@@ -1,9 +1,11 @@
 #!/usr/bin/env python
 """bench.py -- images/sec of VQVAE.forward (enc + VQ + dec) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one VQVAE.forward over one batch of synthetic images per GPU.  Prints ONE JSON line (rank 0).
+--dump-outputs DIR writes what the last timed step of the headline returned (see dump_outputs) so that two builds
+can be compared output for output: the weights and images are seeded, so the same arguments give the same inputs.
 
   headline   BASELINE.json configs[1] (cfg2: B=256 per GPU, 3x32x32, K=512, D=64), per-GPU batch fixed as N grows
              (weak scaling, batch-sharded, no data-path collective).  Convs = tcgen05 kind::tf32 on fp32 activations
@@ -49,6 +51,7 @@ WORKLOADS = {
 }
 HP = dict(h_dim=128, res_h_dim=32, n_res_layers=2)
 METRIC = "images/sec VQVAE fwd (enc+VQ+dec)"
+DUMP_BYTES = 64 << 20          # what --dump-outputs writes in all
 
 
 def load_peaks():
@@ -342,6 +345,35 @@ def capture(model, x):
         return (lambda: model(x)), out, False
 
 
+def step_outputs(model, out):
+    """What a caller of one forward receives, on the host: VQVAE.forward's (loss, x_hat, perplexity) and the model's
+    last_min_encoding_indices (as float64, which holds every index exactly)."""
+    loss, x_hat, perp = out
+    arrays = {"loss": loss, "x_hat": x_hat, "perplexity": perp}
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    arrays["min_encoding_indices"] = model.last_min_encoding_indices.double().cpu().numpy()
+    return arrays
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as <out_dir>/<name>.npy.  Every array gets an equal share of DUMP_BYTES; one that is larger is
+    replaced by a sample of its flattened elements at positions drawn with a fixed seed (the same in every run with the
+    same arguments), in increasing order.  Returns what was written, for the JSON line."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    info = {}
+    for name, a in arrays.items():
+        entry = {"shape": list(a.shape), "dtype": str(a.dtype)}
+        keep = share // a.itemsize
+        if a.size > keep:
+            pos = np.sort(np.random.RandomState(0).choice(a.size, keep, replace=False))
+            a = a.reshape(-1)[pos]
+            entry["sampled_elements"] = keep
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        info[name] = entry
+    return info
+
+
 def oracle_flips(wl, x_np, idx_dev, sd, n_img):
     """Index flips of the timed mode against the C oracle on the first n_img images of the batch (rank 0, untimed)."""
     try:
@@ -370,7 +402,11 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--quick", action="store_true", help="headline only: no fp32 mode, cfg3, cfg5, vq_sweep")
     ap.add_argument("--no-extra-modes", action="store_true", help="alias of --quick")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline's outputs of its last timed step as DIR/<name>.npy (rank 0's shard)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3)
     args.quick = args.quick or args.no_extra_modes
     wl = WORKLOADS[args.workload]
@@ -434,15 +470,17 @@ def main():
         return sorted(rows, key=lambda r: -r["share"])
 
     def device_time(step, steps):
+        """(device ms of `steps` steps, what the last step returned)."""
         evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         barrier()
+        out = None
         for s0, s1 in evs:
             flush.zero_()
             s0.record()
-            step()
+            out = step()
             s1.record()
         barrier()
-        return sum(a.elapsed_time(b) for a, b in evs)
+        return sum(a.elapsed_time(b) for a, b in evs), out
 
     # =============================================================== headline workload
     B, S, K, D = wl["batch"], wl["size"], wl["K"], wl["D"]
@@ -471,8 +509,10 @@ def main():
             step()
         barrier()
         clocks = ClockSampler(local_rank if (full and not os.environ.get("VQB_BENCH_NOSAMPLER")) else -1)
-        dev_ms = device_time(step, args.steps)
+        dev_ms, last = device_time(step, args.steps)
         res = dict(launches=int(launches_per_step * args.steps), graph=is_graph)
+        if full and args.dump_outputs and rank == 0:
+            res["outputs"] = step_outputs(model, last)       # before anything below runs the model again
         if full:
             # ---- end to end: host buffers, copies inside the timed region ----
             xh_host = torch.empty((B, 3, S, S), dtype=torch.float32).pin_memory()
@@ -534,6 +574,9 @@ def main():
 
     main_mode = run_mode(prec_main, True)
     line_extra = {}
+    if "outputs" in main_mode:
+        line_extra["outputs"] = {"dir": os.path.abspath(args.dump_outputs),
+                                 "arrays": dump_outputs(args.dump_outputs, main_mode.pop("outputs"))}
     if not args.quick and prec_main != "fp32" and args.workload == "cfg2":
         m = run_mode("fp32", False)
         line_extra["fp32_mode"] = {"value": m["value"], "unit": "images/sec", "ms_per_step": m["ms_per_step"], "dtype": "f32",
@@ -579,7 +622,7 @@ def main():
         for _ in range(3):
             step()
         nsteps = max(3, min(args.steps, 10))
-        ms, = allmax([device_time(step, nsteps)])
+        ms, = allmax([device_time(step, nsteps)[0]])
         o = {"workload": w["desc"], "dtype": "bf16", "per_gpu_batch": per_gpu_batch, "n_gpus": world, "steps": nsteps,
              "value": per_gpu_batch * world * nsteps / (ms * 1e-3), "unit": "images/sec", "ms_per_step": ms / nsteps,
              "launch": "cuda-graph replay" if is_graph else "eager", "l2": "flushed between timed steps"}

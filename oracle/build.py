@@ -18,10 +18,14 @@ def build(force: bool = False) -> str:
             and os.path.getmtime(_OUT) >= os.path.getmtime(_SRC)):
         return _OUT
     os.makedirs(_OUT_DIR, exist_ok=True)
+    # Processes that build at once (the spawned workers of tests/test_dist_cpu.py on a fresh tree) each compile to
+    # their own file and rename it into place, so none of them can load a library another one is still writing.
+    tmp = f"{_OUT}.{os.getpid()}.tmp"
     # -ffp-contract=off: the restatement spells out every fmaf itself.
     cmd = ["gcc", "-O2", "-std=c11", "-fPIC", "-shared", "-fopenmp",
-           "-ffp-contract=off", "-fno-fast-math", "-o", _OUT, _SRC, "-lm"]
+           "-ffp-contract=off", "-fno-fast-math", "-o", tmp, _SRC, "-lm"]
     subprocess.run(cmd, check=True)
+    os.replace(tmp, _OUT)
     return _OUT
 
 

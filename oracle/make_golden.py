@@ -43,12 +43,25 @@ MODEL_CASES = {
     "k1024_s64": dict(h_dim=128, res_h_dim=32, n_res_layers=2, n_embeddings=1024,
                       embedding_dim=64, codebook="normal", codebook_scale=0.05,
                       batch=2, size=64, wseed=8, xseed=9),
-    # BASELINE configs[2] (cfg3) at its real image size: 256x256, K=1024 (B=2 instead of 128).  z_q is not stored
-    # (it is fl(z_e + fl(E[idx] - z_e)) of the stored z_e / idx, quantizer.py:67) to keep the fixture small.
+    # BASELINE configs[2] (cfg3) at its real image size: 256x256, K=1024 (B=2 instead of 128).  Its full z_e and x_hat
+    # take 3.5 MB, so the fixture keeps idx, hist, loss and perplexity of the whole forward and z_e / x_hat of one
+    # window (see window()), plus the reference's VQ step and decoder run on that window of z_e.
     "cfg3_s256": dict(h_dim=128, res_h_dim=32, n_res_layers=2, n_embeddings=1024,
                       embedding_dim=64, codebook="normal", codebook_scale=0.05,
-                      batch=2, size=256, wseed=18, xseed=19, drop=["z_q"]),
+                      batch=2, size=256, wseed=18, xseed=19, window=[1, 40, 0, 16]),
 }
+
+
+def window(a, case):
+    """The part of a full-size NCHW output of a model case that its fixture stores.  All of it, unless the case has a
+    ``window`` [image, y0, x0, n]: then image ``image``, latent rows and columns [y0, y0 + n) (x0 likewise), scaled to
+    the resolution of ``a`` (z_e is at 1/4 of the image size, x_hat at the full size)."""
+    if "window" not in case:
+        return a
+    i, y0, x0, n = case["window"]
+    s = a.shape[2] // (case["size"] // 4)
+    return a[i:i + 1, :, s * y0:s * (y0 + n), s * x0:s * (x0 + n)]
+
 
 # VectorQuantizer-only cases (BASELINE cfg4 grid at a size the CPU finishes in seconds)
 VQ_CASES = {
@@ -94,6 +107,15 @@ with torch.no_grad():
         out = dict(z_e=z_e.numpy(), idx=idx.numpy(), z_q=z_q.numpy(), x_hat=x_hat.numpy(),
                    loss=loss.numpy(), perplexity=perp.numpy(),
                    hist=onehot.sum(0).numpy().astype(np.int32))
+    elif job["kind"] == "window":
+        # the VQ step and the decoder on a window of z_e (the VQ boundary and decoder checks of a windowed case)
+        hp = job["hp"]
+        m = VQVAE(hp["h_dim"], hp["res_h_dim"], hp["n_res_layers"], hp["n_embeddings"],
+                  hp["embedding_dim"], 0.25).eval()
+        m.load_state_dict({k: torch.from_numpy(data[k]) for k in m.state_dict().keys()})
+        loss, z_q, perp, _, idx = m.vector_quantization(torch.from_numpy(data["__z"]))
+        out = dict(vq_idx=idx.numpy(), vq_loss=loss.numpy(), vq_perplexity=perp.numpy(),
+                   dec_x_hat=m.decoder(z_q.clone()).numpy())
     else:
         vq = VectorQuantizer(int(job["K"]), int(job["D"]), 0.25)
         vq.embedding.weight.data.copy_(torch.from_numpy(data["E"]))
@@ -189,8 +211,11 @@ def main():
                              codebook_scale=c["codebook_scale"], **hp)
         x = make_images(c["batch"], c["size"], c["xseed"])
         out = _run_ref(dict(kind="model", hp=hp), dict(sd, __x=x))
-        for k in c.get("drop", []):
-            out.pop(k)
+        if "window" in c:
+            z = np.ascontiguousarray(window(out["z_e"], c))
+            out = dict(_run_ref(dict(kind="window", hp=hp), dict(sd, __z=z)), z_e=z, idx=out["idx"],
+                       x_hat=np.ascontiguousarray(window(out["x_hat"], c)), loss=out["loss"],
+                       perplexity=out["perplexity"], hist=out["hist"])
         np.savez_compressed(os.path.join(OUT, name + ".npz"), case=json.dumps(c), **out)
         print(name, {k: v.shape for k, v in out.items()}, "codes used", int((out["hist"] > 0).sum()))
     for name, c in VQ_CASES.items():

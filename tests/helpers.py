@@ -4,7 +4,7 @@ import os
 
 import numpy as np
 
-from oracle.make_golden import MODEL_CASES, VQ_CASES, make_vq_inputs  # noqa: F401
+from oracle.make_golden import MODEL_CASES, VQ_CASES, make_vq_inputs, window  # noqa: F401
 from oracle.weights import make_images, make_state_dict
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -12,9 +12,15 @@ HP_KEYS = ("h_dim", "res_h_dim", "n_res_layers", "n_embeddings", "embedding_dim"
 
 
 def load_golden(name):
+    """A golden case.  Model cases also carry the reference's VQ step on the stored z_e (vq_idx, vq_loss,
+    vq_perplexity) and its decoder on the resulting z_q (dec_x_hat): for a full-size fixture these are the forward's
+    own idx, loss, perplexity and x_hat; a windowed fixture (cfg3_s256) stores them for its window."""
     with np.load(os.path.join(GOLDEN, name + ".npz")) as d:
         out = {k: d[k] for k in d.files}
     out["case"] = json.loads(str(out["case"]))
+    if "z_e" in out:
+        for k, full in (("vq_idx", "idx"), ("vq_loss", "loss"), ("vq_perplexity", "perplexity"), ("dec_x_hat", "x_hat")):
+            out.setdefault(k, out[full])
     return out
 
 
@@ -37,15 +43,16 @@ def build_model(hp, sd, device="cuda"):
 
 
 def expected_zq(g, E=None):
-    """The reference's z_q (NCHW) of a golden case, or None when only its hash is stored.  Cases that drop z_q to
-    stay small (cfg3_s256) hold z_e and idx, from which z_q = fl(z_e + fl(E[idx] - z_e)) follows (quantizer.py:60,67)."""
+    """The reference's z_q (NCHW) of a golden case, or None when only its hash is stored.  Cases that do not store z_q
+    to stay small (cfg3_s256) hold z_e and vq_idx, from which z_q = fl(z_e + fl(E[idx] - z_e)) follows
+    (quantizer.py:60,67)."""
     if "z_q" in g:
         return g["z_q"]
     if "z_e" in g and E is not None:
         z = g["z_e"]
         B, D, H, W = z.shape
         rows = np.ascontiguousarray(z.transpose(0, 2, 3, 1)).reshape(-1, D)
-        e = np.asarray(E, dtype=np.float32)[g["idx"].ravel()]
+        e = np.asarray(E, dtype=np.float32)[g["vq_idx"].ravel()]
         zq = (rows + (e - rows).astype(np.float32)).astype(np.float32)
         return np.ascontiguousarray(zq.reshape(B, H, W, D).transpose(0, 3, 1, 2))
     return None

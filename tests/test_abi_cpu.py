@@ -162,7 +162,7 @@ def test_product_never_imports_the_oracle():
                     assert not re.search(r"^\s*(from|import)\s+oracle\b", src, flags=re.M), os.path.join(root, f)
 
 
-def test_reference_checkpoint_loads_on_cpu():
+def test_reference_checkpoint_loads_on_cpu(tmp_path):
     """vqvae_b200.load_checkpoint reads the reference's {'model','results','hyperparameters'} file (utils.py:106-115; written by
     oracle/make_golden.py from the unmodified reference model): architecture from the hyper-parameters, all 23 keys loaded."""
     import numpy as np
@@ -178,15 +178,11 @@ def test_reference_checkpoint_loads_on_cpu():
         assert np.array_equal(got[k].numpy(), v), k
     assert len(m.encoder.conv_stack[5].stack) == hp["n_res_layers"] and not m.training
     # save_checkpoint writes the same format back
-    out = os.path.join(ROOT, "tests", "golden", "_roundtrip.pth")
-    try:
-        vqvae_b200.save_checkpoint(m, data["results"], data["hyperparameters"], out)
-        m2, d2 = vqvae_b200.load_checkpoint(out, device="cpu")
-        assert all(torch.equal(a, b) for a, b in zip(m.state_dict().values(), m2.state_dict().values()))
-        assert d2["hyperparameters"] == data["hyperparameters"]
-    finally:
-        if os.path.exists(out):
-            os.remove(out)
+    out = str(tmp_path / "roundtrip.pth")
+    vqvae_b200.save_checkpoint(m, data["results"], data["hyperparameters"], out)
+    m2, d2 = vqvae_b200.load_checkpoint(out, device="cpu")
+    assert all(torch.equal(a, b) for a, b in zip(m.state_dict().values(), m2.state_dict().values()))
+    assert d2["hyperparameters"] == data["hyperparameters"]
 
 
 def test_convt_out_scatter_column_layout():

@@ -11,7 +11,7 @@ import torch
 
 from oracle import cref
 from tests.helpers import (MODEL_CASES, VQ_CASES, assert_zq_matches, build_model, expected_zq, load_golden,
-                           make_vq_inputs, model_case_inputs)
+                           make_vq_inputs, model_case_inputs, window)
 
 pytestmark = pytest.mark.gpu
 
@@ -241,17 +241,17 @@ def test_vqvae_forward_vs_reference_golden(name):
     xc = _cuda(x)
     # piecewise API the notebook uses (visualization.ipynb cell 1 `reconstruct`)
     z_e = m.pre_quantization_conv(m.encoder(xc.clone()))
-    np.testing.assert_allclose(z_e.cpu().numpy(), g["z_e"], atol=CONV_ATOL, rtol=0)
+    np.testing.assert_allclose(window(z_e.cpu().numpy(), g["case"]), g["z_e"], atol=CONV_ATOL, rtol=0)
     # VQ boundary: the reference's own z_e in -> bit-exact indices, bitwise z_q
     loss_b, zq_b, perp_b, _, idx_b = m.vector_quantization(_cuda(g["z_e"]))
-    assert np.array_equal(idx_b.cpu().numpy(), g["idx"])
+    assert np.array_equal(idx_b.cpu().numpy(), g["vq_idx"])
     E_np = sd["vector_quantization.embedding.weight"]
     assert_zq_matches(g, zq_b.cpu().numpy(), E_np)
-    np.testing.assert_allclose(loss_b.item(), g["loss"], rtol=1e-5)
-    np.testing.assert_allclose(perp_b.item(), g["perplexity"], rtol=2e-5)
+    np.testing.assert_allclose(loss_b.item(), g["vq_loss"], rtol=1e-5)
+    np.testing.assert_allclose(perp_b.item(), g["vq_perplexity"], rtol=2e-5)
     # decoder on the reference's z_q
     xh_b = m.decoder(_cuda(expected_zq(g, E_np)))
-    np.testing.assert_allclose(xh_b.cpu().numpy(), g["x_hat"], atol=CONV_ATOL, rtol=0)
+    np.testing.assert_allclose(xh_b.cpu().numpy(), g["dec_x_hat"], atol=CONV_ATOL, rtol=0)
     # fused forward
     loss, x_hat, perp = m(xc)
     idx = m.last_min_encoding_indices.cpu().numpy()
@@ -267,7 +267,7 @@ def test_vqvae_forward_vs_reference_golden(name):
         assert np.all(gap <= 4 * np.spacing(np.float32(np.abs(d[bad]).max()))), (mism, gap)
     assert mism <= max(1, idx.size // 1000)
     if mism == 0:
-        np.testing.assert_allclose(x_hat.cpu().numpy(), g["x_hat"], atol=CONV_ATOL, rtol=0)
+        np.testing.assert_allclose(window(x_hat.cpu().numpy(), g["case"]), g["x_hat"], atol=CONV_ATOL, rtol=0)
         np.testing.assert_allclose(loss.item(), g["loss"], rtol=1e-5)
         np.testing.assert_allclose(perp.item(), g["perplexity"], rtol=2e-5)
     assert x_hat.shape == x.shape and x_hat.is_contiguous() and x_hat.dtype == torch.float32

@@ -6,7 +6,7 @@ import torch
 
 from oracle import cref, torch_port
 from tests.helpers import (MODEL_CASES, VQ_CASES, assert_zq_matches, expected_zq, load_golden, make_vq_inputs,
-                           model_case_inputs)
+                           model_case_inputs, window)
 
 
 @pytest.mark.parametrize("name", sorted(VQ_CASES))
@@ -38,14 +38,14 @@ def test_c_oracle_model_matches_reference(name):
     g = load_golden(name)
     hp, sd, x = model_case_inputs(g["case"])
     o = cref.vqvae_forward(x, sd, hp["n_res_layers"])
-    np.testing.assert_allclose(o["z_e"], g["z_e"], atol=2e-7, rtol=0)
+    np.testing.assert_allclose(window(o["z_e"], g["case"]), g["z_e"], atol=2e-7, rtol=0)
     # VQ boundary: same z_e in -> identical indices and bitwise z_q
     b = cref.vq_nchw(g["z_e"], sd["vector_quantization.embedding.weight"])
-    assert np.array_equal(b["idx"], g["idx"])
+    assert np.array_equal(b["idx"], g["vq_idx"])
     assert_zq_matches(g, b["zq_nchw"], sd["vector_quantization.embedding.weight"])
     # end to end (oracle convs accumulate in double, the reference in fp32)
     assert np.array_equal(o["idx"], g["idx"])
-    np.testing.assert_allclose(o["x_hat"], g["x_hat"], atol=2e-7, rtol=0)
+    np.testing.assert_allclose(window(o["x_hat"], g["case"]), g["x_hat"], atol=2e-7, rtol=0)
     np.testing.assert_allclose(o["loss"], g["loss"], rtol=1e-5)
     np.testing.assert_allclose(o["perplexity"], g["perplexity"], rtol=2e-5)
 
@@ -58,7 +58,7 @@ def test_torch_port_matches_reference(name):
     tsd = {k: torch.from_numpy(np.array(v)) for k, v in sd.items()}
     o = torch_port.vqvae_forward(torch.from_numpy(x), tsd, hp["n_res_layers"], intermediates=True)
     assert np.array_equal(o["idx"].numpy(), g["idx"])
-    np.testing.assert_allclose(o["z_e"].numpy(), g["z_e"], atol=1e-6, rtol=0)
-    np.testing.assert_allclose(o["x_hat"].numpy(), g["x_hat"], atol=1e-6, rtol=0)
+    np.testing.assert_allclose(window(o["z_e"].numpy(), g["case"]), g["z_e"], atol=1e-6, rtol=0)
+    np.testing.assert_allclose(window(o["x_hat"].numpy(), g["case"]), g["x_hat"], atol=1e-6, rtol=0)
     np.testing.assert_allclose(o["loss"].numpy(), g["loss"], rtol=1e-5)
     np.testing.assert_allclose(o["perplexity"].numpy(), g["perplexity"], rtol=1e-5)
