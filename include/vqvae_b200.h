@@ -170,6 +170,28 @@ int vqb_residual_stack_f32(const float *r, const float *w1_packed, const float *
                            float *out, float *scratch, float *tmp, int B, int H, int W, int C,
                            int Cmid, int n_layers, int precision, void *stream);
 
+/* ---- the latent stage as two fused kernels (TF32), encoder.py:35-36 + residual.py + vqvae.py:16-17
+ * and decoder.py:28-33 -----------------------------------------------------------------------------
+ * For latents whose 128-pixel tile holds whole images (W <= 8, H <= 16): one tcgen05 kernel runs the
+ * whole chain with the activation resident in shared memory, bitwise equal to the per-layer calls.
+ * Weights are the vqb_pack_conv_weight_f32 buffers of the layers, biases may be NULL (= 0).
+ * Encoder tail: in = relu(conv 2) NHWC (B,H,W,C) ->
+ *   E3 conv 3x3 C->C +bias, ReLU -> n_res applications of the shared ResidualLayer (w1: C->Cmid 3x3,
+ *   w2: Cmid->C 1x1), each followed by ReLU -> pre-quant 1x1 C->D +bias -> z_e (B*H*W, D) rows.
+ * Decoder head: zq (B*H*W, D) rows ->
+ *   ConvTranspose 3x3 s1 D->C +bias, ReLU -> the residual stack as above -> ConvTranspose k4 s2 p1
+ *   C->Cout +bias, ReLU -> out NHWC (B,2H,2W,Cout).
+ * C == 128, Cmid == 32, D == 64, Cout == 64, 1 <= n_res <= 4; pointers 16-byte aligned.  Other
+ * shapes return VQB_ERR_UNSUPPORTED (the caller then runs the layers one by one).              */
+int vqb_latent_encoder_f32(const float *in, const float *w3_packed, const float *b3,
+                           const float *w1_packed, const float *w2_packed, const float *wq_packed,
+                           const float *bq, float *z_e, int B, int H, int W, int C, int Cmid,
+                           int D, int n_res, void *stream);
+int vqb_latent_decoder_f32(const float *zq, const float *wt1_packed, const float *bt1,
+                           const float *w1_packed, const float *w2_packed, const float *wt2_packed,
+                           const float *bt2, float *out, int B, int H, int W, int D, int C,
+                           int Cmid, int Cout, int n_res, void *stream);
+
 /* ---- VectorQuantizer.forward, quantizer.py:45-76 --------------------------------
  * z        (N, D) fp32 pixel rows (= z.permute(0,2,3,1).view(-1, e_dim), :45-46)
  * codebook (K, D) fp32 embedding.weight (:26)

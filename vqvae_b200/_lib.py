@@ -47,6 +47,8 @@ SIGNATURES = {
     "vqb_debug_read_cta_times": (_i, [_vp, _i]),
     "vqb_residual_layer_f32": (_i, [_vp] * 5 + [_i] * 7 + [_vp]),
     "vqb_residual_stack_f32": (_i, [_vp] * 6 + [_i] * 7 + [_vp]),
+    "vqb_latent_encoder_f32": (_i, [_vp] * 8 + [_i] * 7 + [_vp]),
+    "vqb_latent_decoder_f32": (_i, [_vp] * 8 + [_i] * 8 + [_vp]),
     "vqb_conv_bf16_packed_bytes": (_sz, [_i, _i, _i]),
     "vqb_pack_conv_weight_bf16": (_i, [_vp, _vp, _i, _i, _i, _vp]),
     "vqb_conv2d_bf16": (_i, [_vp, _vp, _vp, _vp] + [_i] * 8 + [_vp]),

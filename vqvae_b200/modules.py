@@ -25,7 +25,7 @@ import torch.nn as nn
 from . import ops
 from .dist import reduce_vq_stats
 from ._lib import (CONV_K1, CONV_K3, CONV_K4S2, CONVT_K3, CONVT_K4S2, CONVT_K4S2_OUT, NCHW, NHWC, PRECISIONS,
-                   RES_W2)
+                   RES_W2, TF32)
 
 # Default = what the reference itself computes on a GPU: fp32 tensors, convolutions on tensor cores in TF32 with fp32
 # accumulation (PyTorch's torch.backends.cudnn.allow_tf32 default, SURVEY 2.2), bit-exact fp32 VQ.
@@ -218,6 +218,13 @@ class ResidualStack(nn.Module):
                                   C=c1.in_channels, Cmid=c1.out_channels, n_layers=len(self.stack),
                                   precision=_conv_precision())
 
+    def _shared_layer(self):
+        """(conv 3x3, conv 1x1, n) of the reference's ``[layer] * n`` construction, else None."""
+        if len(self.stack) == 0 or any(l is not self.stack[0] for l in self.stack):
+            return None
+        layer = self.stack[0]
+        return layer.res_block[1], layer.res_block[3], len(self.stack)
+
     def _bf16_ok(self):
         if len(self.stack) == 0:
             return True
@@ -265,19 +272,39 @@ class Encoder(nn.Module):
             ResidualStack(h_dim, h_dim, res_h_dim, n_res_layers),
         )
 
-    def _forward_nhwc(self, x):
-        """x: prepared NCHW fp32 CUDA tensor -> (NHWC activation, B, H, W)."""
+    def _head_nhwc(self, x):
+        """x: prepared NCHW fp32 CUDA tensor -> (NHWC output of conv 2 after its ReLU, B, H, W)."""
         B, _, H, W = x.shape
         cs = self.conv_stack
         h = _run_conv(cs[0], x, B, H, W, in_layout=NCHW, relu=True)
         H, W = h.shape[1], h.shape[2]
         h = _run_conv(cs[2], h, B, H, W, relu=True)
-        H, W = h.shape[1], h.shape[2]
+        return h, B, h.shape[1], h.shape[2]
+
+    def _tail_nhwc(self, h, B, H, W):
+        """conv 4 and the stack, one launch per layer: NHWC in -> NHWC stack output."""
+        cs = self.conv_stack
         # the only consumer of conv 4 is the stack, whose first op is ReLU (or, with an
         # empty stack, its final F.relu): fold that ReLU into this epilogue (Q2/Q3).
         h = _run_conv(cs[4], h, B, H, W, relu=True)
-        h = cs[5]._apply_nhwc(h, B, H, W)
-        return h, B, H, W
+        return cs[5]._apply_nhwc(h, B, H, W)
+
+    def _forward_nhwc(self, x):
+        """x: prepared NCHW fp32 CUDA tensor -> (NHWC activation, B, H, W)."""
+        h, B, H, W = self._head_nhwc(x)
+        return self._tail_nhwc(h, B, H, W), B, H, W
+
+    def _fused_tail(self, h, B, H, W, pq):
+        """conv 4 -> stack -> ``pq`` (the pre-quant 1x1) as one kernel, z_e NHWC out: tf32 arithmetic, a shared-weight
+        stack and a latent whose tiles hold whole images.  None when not covered (the caller runs the layers)."""
+        st = self.conv_stack[5]._shared_layer()
+        if _conv_precision() != TF32 or st is None:
+            return None
+        c1, c2, n = st
+        e3 = self.conv_stack[4]
+        return ops.latent_encoder(h, _PACKED.f32(e3.weight, False), _bias(e3), _PACKED.f32(c1.weight, False),
+                                  _PACKED.f32(c2.weight, False), _PACKED.f32(pq.weight, False), _bias(pq), B=B, H=H,
+                                  W=W, C=e3.in_channels, Cmid=c1.out_channels, D=pq.out_channels, n_res=n)
 
     def _bf16_ok(self):
         cs = self.conv_stack
@@ -322,12 +349,27 @@ class Decoder(nn.Module):
     def _forward_from_nhwc(self, z, B, H, W):
         """z: NHWC (B,H,W,in_dim) -> x_hat NCHW."""
         ics = self.inverse_conv_stack
-        h = _run_conv(ics[0], z, B, H, W, relu=True)     # ReLU of the stack folded in (Q2/Q3)
-        H, W = h.shape[1], h.shape[2]
-        h = ics[1]._apply_nhwc(h, B, H, W)
-        h = _run_conv(ics[2], h, B, H, W, relu=True)
+        h = self._fused_head(z, B, H, W)
+        if h is None:
+            h = _run_conv(ics[0], z, B, H, W, relu=True)     # ReLU of the stack folded in (Q2/Q3)
+            H, W = h.shape[1], h.shape[2]
+            h = ics[1]._apply_nhwc(h, B, H, W)
+            h = _run_conv(ics[2], h, B, H, W, relu=True)
         H, W = h.shape[1], h.shape[2]
         return _run_conv(ics[4], h, B, H, W, out_layout=NCHW)
+
+    def _fused_head(self, z, B, H, W):
+        """convT 0 -> stack -> convT 2 (+ReLU) as one kernel: tf32 arithmetic, a shared-weight stack and a latent whose
+        tiles hold whole images.  None when not covered (the caller runs the layers)."""
+        ics = self.inverse_conv_stack
+        st = ics[1]._shared_layer()
+        if _conv_precision() != TF32 or st is None:
+            return None
+        c1, c2, n = st
+        return ops.latent_decoder(z, _PACKED.f32(ics[0].weight, True), _bias(ics[0]), _PACKED.f32(c1.weight, False),
+                                  _PACKED.f32(c2.weight, False), _PACKED.f32(ics[2].weight, True), _bias(ics[2]), B=B,
+                                  H=H, W=W, D=ics[0].in_channels, C=ics[0].out_channels, Cmid=c1.out_channels,
+                                  Cout=ics[2].out_channels, n_res=n)
 
     def _bf16_ok(self):
         ics = self.inverse_conv_stack
@@ -494,8 +536,11 @@ class VQVAE(nn.Module):
             z_e = ops.conv2d_bf16(h, _PACKED.bf16(pq.weight, CONV_K1), _bias(pq), B=B, Cin=pq.in_channels, H=H, W=W,
                                   Cout=pq.out_channels, kind=CONV_K1, relu=False, out_f32=True)   # fp32: feeds the exact VQ
             return z_e, B, H, W
-        h, B, H, W = self.encoder._forward_nhwc(x)
-        z_e = _run_conv(self.pre_quantization_conv, h, B, H, W)              # NHWC (B,H,W,D)
+        h, B, H, W = self.encoder._head_nhwc(x)
+        z_e = self.encoder._fused_tail(h, B, H, W, self.pre_quantization_conv)
+        if z_e is None:
+            h = self.encoder._tail_nhwc(h, B, H, W)
+            z_e = _run_conv(self.pre_quantization_conv, h, B, H, W)          # NHWC (B,H,W,D)
         return z_e, B, H, W
 
     def forward(self, x, verbose=False):

@@ -233,6 +233,42 @@ def residual_stack(r, w1_packed, w2_packed, *, B, H, W, C, Cmid, n_layers, preci
     return out
 
 
+def _ptr(t):
+    return t.data_ptr() if t is not None else None
+
+
+def latent_encoder(h, w3, b3, w1, w2, wq, bq, *, B, H, W, C, Cmid, D, n_res):
+    """E3 conv 3x3 + ReLU -> residual stack -> pre-quant 1x1 as ONE kernel (vqb_latent_encoder_f32): NHWC
+    relu(conv 2) in, z_e NHWC (B, H, W, D) = the VQ's rows out.  None when the shape is not covered (the caller runs
+    the layers)."""
+    _require_cuda(h, "input")
+    z_e = torch.empty((B, H, W, D), dtype=torch.float32, device=h.device)
+    span = _Span(f"latent enc {C}->{Cmid}->{D} x{n_res} {H}x{W}")
+    rc = lib().vqb_latent_encoder_f32(h.data_ptr(), w3.data_ptr(), _ptr(b3), w1.data_ptr(), w2.data_ptr(), wq.data_ptr(),
+                                      _ptr(bq), z_e.data_ptr(), B, H, W, C, Cmid, D, n_res, _stream())
+    if rc == -2:            # VQB_ERR_UNSUPPORTED: nothing was launched
+        return None
+    check(rc, "latent_encoder")
+    span.done()
+    return z_e
+
+
+def latent_decoder(zq, wt1, bt1, w1, w2, wt2, bt2, *, B, H, W, D, C, Cmid, Cout, n_res):
+    """ConvT 3x3 + ReLU -> residual stack -> ConvT k4s2 + ReLU as ONE kernel (vqb_latent_decoder_f32): z_q rows in,
+    NHWC (B, 2H, 2W, Cout) out.  None when the shape is not covered (the caller runs the layers)."""
+    _require_cuda(zq, "input")
+    out = torch.empty((B, 2 * H, 2 * W, Cout), dtype=torch.float32, device=zq.device)
+    span = _Span(f"latent dec {D}->{C}->{Cout} x{n_res} {H}x{W}")
+    rc = lib().vqb_latent_decoder_f32(zq.data_ptr(), wt1.data_ptr(), _ptr(bt1), w1.data_ptr(), w2.data_ptr(),
+                                      wt2.data_ptr(), _ptr(bt2), out.data_ptr(), B, H, W, D, C, Cmid, Cout, n_res,
+                                      _stream())
+    if rc == -2:
+        return None
+    check(rc, "latent_decoder")
+    span.done()
+    return out
+
+
 def vq_forward(z_rows, codebook, defer=False):
     """Fused VectorQuantizer core on (N,D) rows -> (idx int64 (N,), zq (N,D), sse f64 (1,),
     hist int32 (K,)).  defer=True (vqb_vq_forward_deferred_f32) additionally returns the workspace:
