@@ -205,6 +205,8 @@ latent_tc_kernel(const __grid_constant__ CUtensorMap tma_in, const __grid_consta
             float4 *z = reinterpret_cast<float4 *>(sm + b * hs);
             for (int i = tid - 128; i < hs / 16; i += 256) z[i] = make_float4(0.f, 0.f, 0.f, 0.f);
         }
+        // every thread's zeros land before any thread writes its own rows of those buffers (first EPI_ACT below)
+        if (p.nin < NBUF) ptx::named_bar_sync(1, 256);
         for (int g = 0; g < p.ngroups; ++g) {
             const LatGroup G = p.grp[g];
             ptx::mbar_wait_sleep(accfull(g), 0);
