@@ -19,7 +19,7 @@
  *     SURVEY.md 8e): the opt-in shared-memory size of each kernel is configured once
  *     per process, on the device that is current at its first launch; calls may come
  *     from any host thread but are not re-entrant on the same workspace;
- *   - host pointers appear only in vqb_memcpy_async and the vqb_debug_* readers;
+ *   - host pointers appear only in vqb_device_info and vqb_memcpy_async;
  *   - return value: 0 = success, >0 = cudaError_t, <0 = vqb_status below; no C++
  *     exception crosses the boundary;
  *   - activations between layers are NHWC ("pixel rows": (B*H*W, C) row-major); the
@@ -36,7 +36,7 @@
 extern "C" {
 #endif
 
-#define VQB_ABI_VERSION 2
+#define VQB_ABI_VERSION 3
 
 enum vqb_status {
     VQB_OK = 0,
@@ -59,8 +59,8 @@ enum vqb_precision {
 };
 
 int vqb_abi_version(void);
-/* 0: release library -- never reads the environment, no diagnostic / work-skipping code paths
- * compiled in.  1: built with -DVQB_DIAG=1 (tools/diag experiments only).                  */
+/* 0: release library.  1: built with -DVQB_DIAG=1, which adds the in-kernel timelines of
+ * tools/diag and computes the same results.  Neither reads the environment.               */
 int vqb_diag_build(void);
 const char *vqb_error_string(int code);
 /* SM count and compute capability of the current device. */
@@ -128,7 +128,7 @@ int vqb_conv2d_bf16(const void *in, const void *packed, const float *bias, void 
 int vqb_conv_in_bf16(const float *x, const float *w_packed, const float *bias, void *out, int B,
                      int H, int W, int Cout, int relu, void *stream);
 /* VectorQuantizer core for the bf16 pipeline: as vqb_vq_forward_deferred_f32 (fp32 z, bit-exact
- * idx, deferred SSE) but zq is written as bf16 rows (N, D); D == 64 only.                    */
+ * idx, deferred SSE) but zq is written as bf16 rows (N, D); D == 64 and K <= 8192 only.      */
 int vqb_vq_forward_bf16zq_f32(const float *z, const float *codebook, int64_t N, int K, int D,
                               int64_t *idx, void *zq_bf16, double *sse, int32_t *hist,
                               void *workspace, size_t workspace_bytes, void *stream);
@@ -222,16 +222,9 @@ int vqb_vq_reduce_sse_f32(const void *workspace, int64_t N, int K, int D, double
 
 /* Kernel choice of vqb_vq_forward_f32: 0 = auto (tcgen05 kernel when D == 64 and K <= 8192,
  * else the exact FFMA kernel), 1 = always the FFMA kernel, 2 = require the tcgen05 kernel
- * (vq2.cu), 3 = the round-1 tcgen05 kernel (vq_tc.cu, kept for comparison).  All produce
- * bit-identical idx / zq; the switch exists for tests and benchmarks.                 */
+ * (vq2.cu; VQB_ERR_UNSUPPORTED outside its domain).  Both produce bit-identical idx / zq;
+ * the switch exists for tests and benchmarks.                                         */
 int vqb_set_vq_kernel(int which);
-
-/* Diagnostic twin of vqb_vq_forward_f32 (tcgen05 kernel only): additionally dumps the
- * approximate TF32 scores s = ||e||^2 - 2 z.e as (N, ceil(K/256)*256) floats.        */
-int vqb_debug_vq_scores_f32(const float *z, const float *codebook, int64_t N, int K, int D,
-                            int64_t *idx, float *zq, double *sse, int32_t *hist,
-                            void *workspace, size_t workspace_bytes, float *scores,
-                            void *stream);
 
 /* ---- backward of VectorQuantizer.forward, quantizer.py:63-67 (training-mode callers, main.py:74-79) ----
  * g_zq (N,D) = gradient arriving at the returned z_q (straight-through: passes to z unchanged), g_loss = device
@@ -263,15 +256,6 @@ int vqb_gather_rows_f32(const int64_t *idx, const float *codebook, int64_t N, in
 /* In-place ReLU over n floats: the nn.ReLU(True) of residual.py:19, which mutates
  * the caller's tensor when a ResidualLayer is called directly (SURVEY Q2).         */
 int vqb_relu_f32(float *x, int64_t n, void *stream);
-
-/* Diagnostic: copy the first n (<= 32) entries of the in-kernel timeline (globaltimer ns of CTA 0
- * of the last fused residual kernel) to host memory.  Synchronises the device.          */
-int vqb_debug_read_trace(unsigned long long *dst, int n);
-/* Same for the tcgen05 VQ kernel (epilogue warp 4 of CTA 0, local tiles 1-2, 16 marks each; enabled with
- * the environment variable VQB_TC_FLAGS=8).                                                              */
-int vqb_debug_read_trace_vq(unsigned long long *dst, int n);
-/* Per-CTA (start, end<<10 | smid) globaltimer pairs of the last traced tcgen05 VQ launch.               */
-int vqb_debug_read_cta_times(unsigned long long *dst, int n);
 
 /* ---- layout changes at the module boundary (quantizer.py:45, :74) ---------------- */
 int vqb_nchw_to_nhwc_f32(const float *in, float *out, int B, int C, int H, int W, void *stream);

@@ -17,7 +17,7 @@ def _header_functions():
     return sorted(set(re.findall(r"\b(vqb_[a-z0-9_]+)\s*\(", src)))
 
 
-def test_library_builds_loads_and_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_at_abi_version_3():
     from vqvae_b200.build import build
     lib = ctypes.CDLL(build())
     names = _header_functions()
@@ -25,7 +25,7 @@ def test_library_builds_loads_and_exports_every_declared_symbol():
     for n in names:
         assert hasattr(lib, n), f"{n} declared in include/vqvae_b200.h but not exported"
     lib.vqb_abi_version.restype = ctypes.c_int
-    assert lib.vqb_abi_version() == 2
+    assert lib.vqb_abi_version() == 3
     assert lib.vqb_diag_build() == 0          # the shipped library never reads the environment
     lib.vqb_error_string.restype = ctypes.c_char_p
     assert b"workspace" in lib.vqb_error_string(-3)
@@ -121,8 +121,9 @@ def test_default_precision_is_the_reference_gpu_arithmetic():
         vqvae_b200.set_precision("fp8")
 
 
-def test_new_entry_points_validate_arguments_without_a_gpu():
-    """bf16 pipeline entry points: bad arguments / unsupported shapes are rejected before any CUDA call."""
+def test_entry_points_and_vq_kernel_choice_validate_arguments_without_a_gpu():
+    """bf16 pipeline entry points and the VQ kernel choice: bad arguments / unsupported shapes are rejected before any
+    CUDA call."""
     from vqvae_b200 import _lib
     lib = _lib.lib()
     buf = (ctypes.c_float * 64)()
@@ -141,7 +142,7 @@ def test_new_entry_points_validate_arguments_without_a_gpu():
     # the fp32-activation entry points refuse the bf16 enum instead of silently running TF32 (round-1 verdict)
     assert lib.vqb_conv2d_f32(p, p, None, None, p, 1, 64, 8, 8, 64, 3, 3, 1, 1, 0, 1, 1, 0, _lib.BF16, None) == -2
     assert lib.vqb_residual_layer_f32(p, p, p, p, p, 1, 8, 8, 32, 32, 1, _lib.BF16, None) == -2
-    assert lib.vqb_set_vq_kernel(3) == 0 and lib.vqb_set_vq_kernel(0) == 0
+    assert lib.vqb_set_vq_kernel(3) == -1 and lib.vqb_set_vq_kernel(0) == 0
 
 
 def test_no_cpu_fallback():

@@ -196,6 +196,35 @@ def test_bf16_model_forward_tolerance(name):
         np.testing.assert_allclose(window(x_hat.cpu().numpy(), g["case"]), g["x_hat"], atol=3e-3, rtol=0)
 
 
+def test_bf16_mode_beyond_the_vq_kernel_runs_tf32():
+    """The bf16 pipeline's VQ (z_q written as bf16 rows) exists on the tcgen05 kernel only, K <= 8192.  A bf16-mode
+    model with a larger codebook warns once and runs the TF32 kernels: bitwise its tf32-mode forward."""
+    import warnings
+    import vqvae_b200
+    from models.vqvae import VQVAE
+    from vqvae_b200.synth import make_images, make_state_dict
+    with vqvae_b200.precision("bf16"):
+        assert VQVAE(128, 32, 2, 8192, 64, 0.25)._bf16_pipeline()
+    sd = make_state_dict(128, 32, 2, 9000, 64, seed=0, codebook="normal", codebook_scale=0.05)
+    m = VQVAE(128, 32, 2, 9000, 64, 0.25)
+    m.load_state_dict({k: torch.from_numpy(np.array(v)) for k, v in sd.items()})
+    m = m.cuda().eval()
+    x = torch.from_numpy(make_images(3, 32, seed=1)).cuda()
+    out = {}
+    with torch.no_grad():
+        for mode in ("tf32", "bf16"):
+            with vqvae_b200.precision(mode), warnings.catch_warnings(record=True) as caught:
+                warnings.simplefilter("always")
+                loss, x_hat, perp = m(x.clone())
+                m(x.clone())
+            torch.cuda.synchronize()
+            out[mode] = (loss.item(), x_hat.cpu(), perp.item(), m.last_min_encoding_indices.cpu())
+            msgs = [str(w.message) for w in caught if "no bf16 kernels" in str(w.message)]
+            assert len(msgs) == (1 if mode == "bf16" else 0), msgs
+    (l_t, x_t, p_t, i_t), (l_b, x_b, p_b, i_b) = out["tf32"], out["bf16"]
+    assert torch.equal(i_b, i_t) and torch.equal(x_b, x_t) and l_b == l_t and p_b == p_t
+
+
 @pytest.mark.parametrize("B,H,W,relu", [(2, 256, 256, True), (5, 32, 32, True), (3, 64, 64, False), (2, 16, 16, True), (1, 12, 20, True), (300, 32, 32, True)])
 def test_bf16_input_conv_vs_oracle(B, H, W, relu):
     """encoder.py:29-31 in the bf16 pipeline: fp32 NCHW image -> bf16 NHWC.  The 48-tap contraction runs as kind::tf32 on the

@@ -27,5 +27,5 @@ for i, (w, g) in enumerate(zip(want, got)):
     same = w[0] == g[1] and torch.equal(w[1], g[2]) and w[2] == g[3]
     alias = [j for j, ww in enumerate(want) if ww[0] == g[1]]
     xalias = [j for j, ww in enumerate(want) if torch.equal(ww[1], g[2])]
-    print(f"PDL={os.environ.get('VQB_PDL','-')} {prec} graph={use_graph} depth={depth} batch {i}: same={same} loss_of={alias} xhat_of={xalias} "
+    print(f"{prec} graph={use_graph} depth={depth} batch {i}: same={same} loss_of={alias} xhat_of={xalias} "
           f"loss {w[0]:.9f} vs {g[1]:.9f}")

@@ -79,7 +79,7 @@ for raw in (False, True):
         t0 = time.perf_counter()
         pipe.run((hosts[i % 3] for i in range(200)), consume)
         dt = time.perf_counter() - t0
-        print(f"raw={raw} MEMCPY_RT={os.environ.get('VQB_MEMCPY_RUNTIME','0')}: {dt/200*1e3:.3f} ms/step  {200*B/dt/1e6:.3f} M img/s")
+        print(f"raw={raw}: {dt/200*1e3:.3f} ms/step  {200*B/dt/1e6:.3f} M img/s")
     # host-side cost of push alone (GPU idle): time 50 pushes then drain
     torch.cuda.synchronize()
     t0 = time.perf_counter()

@@ -42,9 +42,6 @@ SIGNATURES = {
     "vqb_relu_f32": (_i, [_vp, _i64, _vp]),
     "vqb_launch_count": (C.c_ulonglong, []),
     "vqb_set_vq_kernel": (_i, [_i]),
-    "vqb_debug_read_trace": (_i, [_vp, _i]),
-    "vqb_debug_read_trace_vq": (_i, [_vp, _i]),
-    "vqb_debug_read_cta_times": (_i, [_vp, _i]),
     "vqb_residual_layer_f32": (_i, [_vp] * 5 + [_i] * 7 + [_vp]),
     "vqb_residual_stack_f32": (_i, [_vp] * 6 + [_i] * 7 + [_vp]),
     "vqb_latent_encoder_f32": (_i, [_vp] * 8 + [_i] * 7 + [_vp]),
@@ -55,7 +52,6 @@ SIGNATURES = {
     "vqb_conv_in_bf16": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "vqb_vq_forward_bf16zq_f32": (_i, [_vp, _vp, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "vqb_residual_layer_bf16": (_i, [_vp] * 4 + [_i] * 6 + [_vp]),
-    "vqb_debug_vq_scores_f32": (_i, [_vp, _vp, _i64, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _vp]),
 }
 
 
@@ -69,7 +65,7 @@ def lib():
             fn = getattr(handle, name)   # AttributeError if the symbol is missing
             fn.restype = res
             fn.argtypes = args
-        if handle.vqb_abi_version() != 2:
+        if handle.vqb_abi_version() != 3:
             raise RuntimeError("libvqvae_b200.so ABI version mismatch")
         _lib = handle
     return _lib

@@ -1,18 +1,13 @@
 // api.cu -- the extern "C" boundary declared in include/vqvae_b200.h.
-#include <cstdlib>
-
 #include "common.cuh"
 
 size_t vq_exact_workspace_bytes(int K);
 int launch_vq_exact(const float *z, const float *E, long long N, int K, int D, long long *idx, float *zq,
                     double *sse, int *hist, void *ws, cudaStream_t s);
 
-size_t vq_tc_workspace_bytes(int K);
-bool vq_tc_supported(long long N, int K, int D);
+size_t vq2_workspace_bytes(int K);
 size_t vq_ws_marker_offset(int K);
 int launch_vq_reduce_sse(const void *ws, int K, double *sse, cudaStream_t s);
-int launch_vq_tc(const float *z, const float *E, long long N, int K, int D, long long *idx, void *zq, double *sse,
-                 int *hist, void *ws, float *dbg, int defer, int zq_bf16, cudaStream_t s);
 int launch_conv_in_tc_ex(const float *x, const float *wp, const float *bias, void *y, int B, int H, int W, int Cout,
                          int relu, int out_bf16, cudaStream_t s);
 
@@ -40,24 +35,10 @@ int launch_conv_halo(const ConvLaunch &p, const float *w_tc, cudaStream_t s);
 bool conv_tc_supported(const ConvLaunch &p);
 int launch_conv_tc(const ConvLaunch *ph, int nph, const float *w_tc, int total_taps, cudaStream_t s);
 
-int vqb_halo_wp() {
-    static const int wp = [] { const char *e = vqb_getenv("VQB_HALO_WP"); return (e && atoi(e) == 16) ? 16 : 10; }();
-    return wp;
-}
-
-int vqb_pdl_enabled() {
-    static int on = -1;
-    if (on < 0) {
-        const char *e = vqb_getenv("VQB_PDL");
-        on = e ? (atoi(e) != 0) : 1;
-    }
-    return on;
-}
-
 unsigned long long g_vqb_launches = 0;
-static int g_vq_kernel = 0;   // 0 auto, 1 exact FFMA kernel, 2 tcgen05 kernel (vq2.cu), 3 round-1 tcgen05 kernel (vq_tc.cu)
+static int g_vq_kernel = 0;   // 0 auto, 1 exact FFMA kernel, 2 tcgen05 kernel (vq2.cu)
 extern "C" int vqb_set_vq_kernel(int which) {
-    if (which < 0 || which > 3) return VQB_ERR_BAD_ARG;
+    if (which < 0 || which > 2) return VQB_ERR_BAD_ARG;
     g_vq_kernel = which;
     return 0;
 }
@@ -65,7 +46,7 @@ extern "C" unsigned long long vqb_launch_count(void) { return g_vqb_launches; }
 
 extern "C" int vqb_abi_version(void) { return VQB_ABI_VERSION; }
 
-// 0 = release library (never reads the environment, no work-skipping paths compiled in); 1 = diagnostic build
+// 0 = release library; 1 = diagnostic build (adds in-kernel timelines, same results)
 extern "C" int vqb_diag_build(void) { return VQB_DIAG; }
 
 extern "C" const char *vqb_error_string(int code) {
@@ -224,9 +205,9 @@ extern "C" size_t vqb_vq_workspace_bytes(int64_t N, int K, int D) {
     return vq_ws_marker_offset(K) + 256;
 }
 
-// [exact / tcgen05 kernel workspace (whichever is larger)][256 B: deferred-reduction marker]
+// [exact / vq2 kernel workspace (whichever is larger)][256 B: deferred-reduction marker]
 size_t vq_ws_marker_offset(int K) {
-    const size_t a = vq_exact_workspace_bytes(K), b = vq_tc_workspace_bytes(K);
+    const size_t a = vq_exact_workspace_bytes(K), b = vq2_workspace_bytes(K);
     return ((a > b ? a : b) + 255) / 256 * 256;
 }
 
@@ -261,15 +242,11 @@ static int vq_forward_impl(const float *z, const float *codebook, int64_t N, int
     const uintptr_t al = reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(codebook) |
                          reinterpret_cast<uintptr_t>(zq) | reinterpret_cast<uintptr_t>(workspace);
     if (al & 15) return VQB_ERR_ALIGNMENT;
-    const bool tc_ok = vq_tc_supported(N, K, D), v2_ok = vq2_supported(N, K, D);
+    const bool v2_ok = vq2_supported(N, K, D);
     if (g_vq_kernel == 2 && !v2_ok) return VQB_ERR_UNSUPPORTED;
-    if (g_vq_kernel == 3 && !tc_ok) return VQB_ERR_UNSUPPORTED;
-    if (v2_ok && (g_vq_kernel == 0 || g_vq_kernel == 2))
+    if (v2_ok && g_vq_kernel != 1)
         return launch_vq2(z, codebook, N, K, D, reinterpret_cast<long long *>(idx), zq, sse, hist, workspace, defer, 0,
                           (cudaStream_t)stream);
-    if (tc_ok && g_vq_kernel != 1)
-        return launch_vq_tc(z, codebook, N, K, D, reinterpret_cast<long long *>(idx), zq, sse, hist, workspace,
-                            nullptr, defer, 0, (cudaStream_t)stream);
     const int rc = launch_vq_exact(z, codebook, N, K, D, reinterpret_cast<long long *>(idx), zq, sse, hist, workspace,
                                    (cudaStream_t)stream);
     if (rc || !defer) return rc;
@@ -279,7 +256,7 @@ static int vq_forward_impl(const float *z, const float *codebook, int64_t N, int
 }
 
 // VQB_BF16 pipeline: same contract as vqb_vq_forward_deferred_f32 (fp32 z in, bit-exact idx) but z_q leaves as bf16
-// rows for the decoder's first conv; tcgen05 kernel only (D == 64).
+// rows for the decoder's first conv; vq2 kernel only (D == 64, K <= 8192).
 extern "C" int vqb_vq_forward_bf16zq_f32(const float *z, const float *codebook, int64_t N, int K, int D, int64_t *idx,
                                          void *zq_bf16, double *sse, int32_t *hist, void *workspace,
                                          size_t workspace_bytes, void *stream) {
@@ -289,12 +266,9 @@ extern "C" int vqb_vq_forward_bf16zq_f32(const float *z, const float *codebook, 
     const uintptr_t al = reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(codebook) |
                          reinterpret_cast<uintptr_t>(zq_bf16) | reinterpret_cast<uintptr_t>(workspace);
     if (al & 15) return VQB_ERR_ALIGNMENT;
-    if (vq2_supported(N, K, D) && g_vq_kernel != 3)
-        return launch_vq2(z, codebook, N, K, D, reinterpret_cast<long long *>(idx), zq_bf16, sse, hist, workspace, 1, 1,
-                          (cudaStream_t)stream);
-    if (!vq_tc_supported(N, K, D)) return VQB_ERR_UNSUPPORTED;
-    return launch_vq_tc(z, codebook, N, K, D, reinterpret_cast<long long *>(idx), zq_bf16, sse, hist, workspace, nullptr, 1, 1,
-                        (cudaStream_t)stream);
+    if (!vq2_supported(N, K, D)) return VQB_ERR_UNSUPPORTED;
+    return launch_vq2(z, codebook, N, K, D, reinterpret_cast<long long *>(idx), zq_bf16, sse, hist, workspace, 1, 1,
+                      (cudaStream_t)stream);
 }
 
 // encoder.py:29-31 in the VQB_BF16 pipeline: fp32 NCHW image in, bf16 NHWC activation out (Cout == 64); the 48-tap
@@ -309,16 +283,6 @@ extern "C" int vqb_conv_in_bf16(const float *x, const float *w_packed, const flo
         if (rc != VQB_ERR_UNSUPPORTED) return rc;
     }
     return launch_conv_in_tc_ex(x, w_packed, bias, out, B, H, W, Cout, relu, 1, (cudaStream_t)stream);
-}
-
-extern "C" int vqb_debug_vq_scores_f32(const float *z, const float *codebook, int64_t N, int K, int D, int64_t *idx,
-                                       float *zq, double *sse, int32_t *hist, void *workspace,
-                                       size_t workspace_bytes, float *scores, void *stream) {
-    if (!z || !codebook || !idx || !zq || !sse || !hist || !workspace || !scores) return VQB_ERR_BAD_ARG;
-    if (!vq_tc_supported(N, K, D)) return VQB_ERR_UNSUPPORTED;
-    if (workspace_bytes < vqb_vq_workspace_bytes(N, K, D)) return VQB_ERR_WORKSPACE;
-    return launch_vq_tc(z, codebook, N, K, D, reinterpret_cast<long long *>(idx), zq, sse, hist, workspace, scores, 0, 0,
-                        (cudaStream_t)stream);
 }
 
 extern "C" int vqb_residual_layer_f32(const float *r, const float *w1_packed, const float *w2_packed, float *out,
@@ -349,8 +313,7 @@ extern "C" int vqb_residual_stack_f32(const float *r, const float *w1_packed, co
     if (n_layers > 1 && !scratch) return VQB_ERR_BAD_ARG;
     if (precision < VQB_FP32 || precision > VQB_BF16) return VQB_ERR_BAD_ARG;
     if (precision == VQB_BF16) return VQB_ERR_UNSUPPORTED;
-    static const bool fuse = [] { const char *e = vqb_getenv("VQB_RES_FUSE"); return !(e && e[0] == '0'); }();
-    if (fuse && n_layers > 1 && precision != VQB_FP32 && res_tc_supported(C, Cmid, r, out)) {
+    if (n_layers > 1 && precision != VQB_FP32 && res_tc_supported(C, Cmid, r, out)) {
         // all applications in ONE launch: the activation never leaves shared memory between them
         const int rc = launch_res_tc(r, w1_packed + (size_t)9 * C * Cmid, w2_packed + (size_t)C * Cmid, out, B, H, W, C,
                                      Cmid, 1, n_layers, (cudaStream_t)stream);
@@ -385,8 +348,7 @@ extern "C" int vqb_memcpy_async(void *dst, const void *src, size_t bytes, int ki
             p = nullptr;
         return reinterpret_cast<PFN_cuMemcpyAsync>(p);
     }();
-    static const bool use_rt = [] { const char *e = vqb_getenv("VQB_MEMCPY_RUNTIME"); return e && e[0] == '1'; }();
-    if (fn && !use_rt) {
+    if (fn) {
         const int rc = fn((unsigned long long)(uintptr_t)dst, (unsigned long long)(uintptr_t)src, bytes, stream);
         return rc == 0 ? 0 : VQB_ERR_BAD_ARG;
     }

@@ -7,15 +7,15 @@
 
 #define VQB_MAX_TAPS 16
 
-// Experiment / diagnostic knobs (VQB_* environment variables, the work-skipping VQB_TC_FLAGS bits, in-kernel
-// timelines) exist only in a library built with -DVQB_DIAG=1 (VQB_DIAG=1 python -m vqvae_b200.build, used by
-// tools/diag).  The release library never reads the environment: vqb_getenv() is a constant nullptr there and the
-// flag tests in the kernels fold away.
+// The library never reads the environment.  A library built with -DVQB_DIAG=1 (VQB_DIAG=1 python -m
+// vqvae_b200.build, used by tools/diag) differs from the release build only by the in-kernel timelines of vq2,
+// hconv and res_bf16 (#if VQB_DIAG); it computes the same results with the same launches.
 #ifndef VQB_DIAG
 #define VQB_DIAG 0
 #endif
-#include <stdlib.h>
-static inline const char *vqb_getenv(const char *name) { return VQB_DIAG ? getenv(name) : nullptr; }
+
+// halo tile width in pixels of conv_halo.cu / res_tc.cu / latent_tc.cu: an 8-pixel tile + 1 each side
+constexpr int VQB_HALO_WP = 10;
 
 // One launch of the generalised gather-form convolution
 //   out[n, gy*out_step+out_py, gx*out_step+out_px, co] =
@@ -46,9 +46,7 @@ extern unsigned long long g_vqb_launches;
 
 // Programmatic dependent launch: the next kernel of the layer chain may start its prologue (barrier init,
 // TMEM allocation, tensor-map prefetch) while this one drains; it blocks in pdl_wait() until the previous
-// grid has completed and its writes are visible.  VQB_PDL=0 in the environment disables the attribute.
-int vqb_pdl_enabled();
-int vqb_halo_wp();           // halo tile width of conv_halo.cu / res_tc.cu: 10, or 16 with VQB_HALO_WP=16
+// grid has completed and its writes are visible.
 #ifdef __CUDACC__
 #include <utility>
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
@@ -62,7 +60,7 @@ static inline cudaError_t vqb_launch(void (*kernel)(KArgs...), dim3 grid, dim3 b
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = vqb_pdl_enabled() ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 // same, as thread-block clusters of `cluster` CTAs along x (the grid must be a multiple of it)
@@ -77,7 +75,7 @@ static inline cudaError_t vqb_launch_cluster(void (*kernel)(KArgs...), dim3 grid
     attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = vqb_pdl_enabled() ? 2 : 1;
+    cfg.numAttrs = 2;
     return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 #endif

@@ -2,17 +2,13 @@
 //
 // conv_tc.cu fetches the 128-pixel A tile once per tap (9x for a 3x3), which makes the k-loop
 // L2->SM feed bound (profiles/r01: tensor pipe 7-30 % active).  Here the input tile is loaded
-// ONCE per 32-channel chunk, with its 1-pixel halo, as a TMA box {32 ch, 16 px, BN img, BH+2 rows}
+// ONCE per 32-channel chunk, with its 1-pixel halo, as a TMA box {32 ch, WP px, BN img, BH+2 rows}
 // (tensor-map dims ordered c,w,n,h so the rows of the BN images interleave), and the nine taps are
-// nine UMMA shared-memory descriptors into that one tile: tap (dy,dx) starts (dy+1)*BN*16+(dx+1)
-// 128-byte rows further in, 8-pixel row groups stay 16 rows (2048 B) apart, and because the
-// padded row length is a multiple of 8 rows the 128B-swizzle phase of every group is the same
-// (the descriptor's base_offset stays 0: the hardware uses absolute address bits).  Only the
-// weight tiles stream through the ring.
+// nine UMMA shared-memory descriptors into that one tile: tap (dy,dx) starts (dy+1)*BN*WP+(dx+1)
+// 128-byte rows further in and 8-pixel row groups stay WP rows apart (the descriptor's base_offset
+// stays 0: the hardware uses absolute address bits).  Only the weight tiles stream through the ring.
 // Used for encoder.py:35-36, decoder.py:28-29 (ConvTranspose k3s1 = same neighbourhood, tap
 // offsets pad - r) and the 3x3 of residual.py:20.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "ptx.cuh"
 
@@ -24,9 +20,9 @@ constexpr int CH_MAX_STAGES = 32;     // weight-tile ring: as deep as shared mem
 constexpr int CH_GROUP = 4;           // ring stages released per tcgen05.commit (a commit costs ~230 cycles)
 constexpr int CH_HALO_BUFS = 2;       // halo tiles are double buffered: chunk c+2 loads while c+1 computes
 constexpr int CH_MAX_CHUNKS = 8;       // Cin <= 256
-// Halo tile width (p.WP): 8 pixels + 1 each side = 10.  Not a multiple of 8 on purpose: the swizzle phase of a row
-// comes from its absolute address, for TMA and UMMA alike, so an 8-row operand group may start at any row
-// (SBO = WP rows); padding to 16 wasted 37 % of the tile.  VQB_HALO_WP=16 restores the padded layout.
+// Halo tile width (p.WP = VQB_HALO_WP): 8 pixels + 1 each side = 10.  Not a multiple of 8 on purpose: the swizzle phase
+// of a row comes from its absolute address, for TMA and UMMA alike, so an 8-row operand group may start at any row
+// (SBO = WP rows); padding to 16 wasted 37 % of the tile.
 
 struct ConvHaloParams {
     const float *bias, *skip;
@@ -36,7 +32,7 @@ struct ConvHaloParams {
     int stages, relu;
     int nmma;               // MMA issuer warps (1 or 2): k-step i goes to issuer i % nmma, private accumulators summed
                             // by the epilogue in a fixed order (see res_tc.cu)
-    int WP;                 // halo tile width in pixels (10, or 16 with VQB_HALO_WP=16)
+    int WP;                 // halo tile width in pixels (VQB_HALO_WP)
     int shuffle_cout;       // > 0: the GEMM's 16 columns are (py, px, co) of a k4s2p1 transposed conv with this
                             // many real output channels; the epilogue pixel-shuffles them into the NCHW output
     int tap_w[9], tap_dy[9], tap_dx[9];
@@ -281,17 +277,7 @@ int ch_pow2_ceil(int x) {
 
 }  // namespace
 
-int conv_halo_mode() {          // on by default; VQB_CONV_HALO=0 falls back to the per-tap TMA kernel (conv_tc.cu)
-    static int mode = -1;
-    if (mode < 0) {
-        const char *e = vqb_getenv("VQB_CONV_HALO");
-        mode = e ? atoi(e) : 1;
-    }
-    return mode;
-}
-
 bool conv_halo_supported(const ConvLaunch &p) {
-    if (conv_halo_mode() == 0) return false;
     const bool nhwc = p.in_sc == 1 && p.in_sw == p.Cin && p.out_sc == 1 && p.out_sw == p.Cout;
     if (!nhwc || p.ntaps != 9 || p.in_step != 1 || p.out_step != 1 || p.OHg != p.H || p.OWg != p.W) return false;
     for (int t = 0; t < 9; ++t)
@@ -313,10 +299,7 @@ int launch_conv_halo_ex(const ConvLaunch &p, const float *w_tc, int shuffle_cout
     q.tiles_x = (p.W + 7) / 8;
     q.tiles_y = (p.H + q.BH - 1) / q.BH;
     const int tiles_n = (p.B + q.BN - 1) / q.BN;
-    {
-        static const int want = [] { const char *e = vqb_getenv("VQB_CONV_NMMA"); return (e && atoi(e) == 1) ? 1 : 2; }();
-        q.nmma = (want == 2 && 2 * p.Cout <= 256) ? 2 : 1;       // <= 256 TMEM columns: two CTAs per SM can still allocate
-    }
+    q.nmma = 2 * p.Cout <= 256 ? 2 : 1;       // <= 256 TMEM columns: two CTAs per SM can still allocate
     q.shuffle_cout = shuffle_cout;
     for (int t = 0; t < 9; ++t) { q.tap_w[t] = p.tap_w[t]; q.tap_dy[t] = p.tap_dy[t]; q.tap_dx[t] = p.tap_dx[t]; }
 
@@ -324,7 +307,7 @@ int launch_conv_halo_ex(const ConvLaunch &p, const float *w_tc, int shuffle_cout
     // dims ordered (c, w, n, h): the BN images of a tile interleave row by row in shared memory
     const uint64_t dims[4] = {(uint64_t)p.Cin, (uint64_t)p.W, (uint64_t)p.B, (uint64_t)p.H};
     const uint64_t strides[3] = {(uint64_t)p.Cin * 4, (uint64_t)p.H * p.W * p.Cin * 4, (uint64_t)p.W * p.Cin * 4};
-    const int WP = vqb_halo_wp();
+    const int WP = VQB_HALO_WP;
     q.WP = WP;
     const uint32_t box[4] = {32u, (uint32_t)WP, (uint32_t)q.BN, (uint32_t)(q.BH + 2)};
     const uint32_t es[4] = {1u, 1u, 1u, 1u};
@@ -362,7 +345,7 @@ int launch_conv_halo_ex(const ConvLaunch &p, const float *w_tc, int shuffle_cout
 // ConvTranspose2d(Cin -> Cout <= 4, k4 s2 p1), NHWC in -> NCHW out, as ONE 3x3-neighbourhood GEMM with 16 columns
 // (py, px, co): w_shuffle = [9 taps][16][Cin] packed by vqb_pack_conv_weight_f32 (third region).
 bool convt_shuffle_supported(int Cin, int Cout, const void *in, const void *out) {
-    return conv_halo_mode() != 0 && Cin % 32 == 0 && Cin <= 32 * CH_MAX_CHUNKS && Cout >= 1 && Cout <= 4 &&
+    return Cin % 32 == 0 && Cin <= 32 * CH_MAX_CHUNKS && Cout >= 1 && Cout <= 4 &&
            (reinterpret_cast<uintptr_t>(in) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 7) == 0;
 }
 

@@ -289,10 +289,7 @@ int launch_conv_tc(const ConvLaunch *ph, int nph, const float *w_tc, int total_t
     else stages -= stages % CT_GROUP;             // a reused ring must hold whole commit groups
     if (stages < 1) stages = 1;
     q.stages = stages;
-    {
-        static const int want = [] { const char *e = vqb_getenv("VQB_CONV_NMMA"); return (e && atoi(e) == 1) ? 1 : 2; }();
-        q.nmma = (want == 2 && 2 * p.Cout <= 256 && stages >= 2 && (stages % 2 == 0 || stages >= maxk)) ? 2 : 1;
-    }
+    q.nmma = (2 * p.Cout <= 256 && stages >= 2 && (stages % 2 == 0 || stages >= maxk)) ? 2 : 1;
     const int smem = stages * stage_bytes + 192 + p.Cout * 4 + 1024;
     static int attr_max = 0;
     if (smem > attr_max) {

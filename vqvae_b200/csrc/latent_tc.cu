@@ -361,7 +361,7 @@ int lt_pow2_ceil(int x) {
 int lat_geometry(LatParams &q, int B, int H, int W, int *smem) {
     if (W > 8 || H > 16) return VQB_ERR_UNSUPPORTED;
     const int BH = lt_pow2_ceil(H) < 16 ? lt_pow2_ceil(H) : 16;
-    q.B = B; q.H = H; q.W = W; q.BN = 16 / BH; q.WP = vqb_halo_wp();
+    q.B = B; q.H = H; q.W = W; q.BN = 16 / BH; q.WP = VQB_HALO_WP;
     q.in_bytes = (BH + 2) * q.BN * q.WP * 128;
     q.halo_stride = (q.in_bytes + 1023) & ~1023;
     const int fixed = 4 * q.halo_stride + LT_A2 + LT_MAXK * 8 + 256 * 4 + 8 * (2 * LT_MAX_STAGES + 2 * LT_MAXG + 2);

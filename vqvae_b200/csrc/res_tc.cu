@@ -12,24 +12,8 @@
 //          A operand of GEMM2 (one 128-byte row per pixel per 32 channels)
 //   GEMM2  D2[128][C] = A2[128][Cmid] * W2[C][Cmid]^T
 //   epi2   tcgen05.ld D2 -> + r (skip, from global/L2) -> ReLU -> NHWC store
-#include <cstdlib>
-
 #include "common.cuh"
 #include "ptx.cuh"
-
-// in-kernel timeline of CTA 0 (globaltimer ns), read back with vqb_debug_read_trace (diagnostic only)
-__device__ unsigned long long g_vqb_trace[32];
-__device__ __forceinline__ void trace_mark(int i) {
-    if (blockIdx.x == 0) {
-        unsigned long long t;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        g_vqb_trace[i] = t;
-    }
-}
-extern "C" int vqb_debug_read_trace(unsigned long long *dst, int n) {
-    if (!dst || n < 1 || n > 32) return VQB_ERR_BAD_ARG;
-    return vqb_cuda_status(cudaMemcpyFromSymbol(dst, g_vqb_trace, sizeof(unsigned long long) * n));
-}
 
 namespace {
 
@@ -46,7 +30,7 @@ struct ResTcParams {
     int B, H, W, C, Cmid;
     int BH, BN, tiles_x, tiles_y;          // tile = 8 px wide x (BH rows x BN images = 16)
     int stages;
-    int WP;                 // halo tile width in pixels: 8 + 1 each side = 10 (see conv_halo.cu), or 16 (VQB_HALO_WP)
+    int WP;                 // halo tile width in pixels: 8 + 1 each side = VQB_HALO_WP (see conv_halo.cu)
     int relu_out;
     int nprod;              // W1 producer warps (2 in staged mode: warp 5 takes the odd k-steps; one warp issuing a 4 KB
                             // box per k-step behind an mbarrier wait could not keep four MMA issuers fed)
@@ -94,7 +78,6 @@ res_tc_kernel(const __grid_constant__ CUtensorMap tma_in, const __grid_constant_
     volatile uint32_t *tmem_holder = reinterpret_cast<volatile uint32_t *>(sm + bar_off + RT_MISC);
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (tid == 128) trace_mark(0);                     // kernel entry
     int tcols = 32;
     while (tcols < p.nmma * p.Cmid + p.C) tcols <<= 1;
     const uint32_t d2col = (uint32_t)(p.nmma * p.Cmid);     // D1 partials at columns 0.., D2 right after them
@@ -123,7 +106,6 @@ res_tc_kernel(const __grid_constant__ CUtensorMap tma_in, const __grid_constant_
     ptx::tc_fence_after();
     const uint32_t tmem_base = *tmem_holder;
     pdl_launch_dependents();       // the next layer may start its prologue (it blocks in its own pdl_wait)
-    if (tid == 128) trace_mark(1);                     // barriers + TMEM ready
 
 
     // ---- epilogue 2 of the staged layout, columns [c_beg, c_end) of this thread's row: D2 + skip (centre tap of
@@ -274,7 +256,6 @@ res_tc_kernel(const __grid_constant__ CUtensorMap tma_in, const __grid_constant_
                 for (int c = 0; issuer && c < chunks; ++c, kbase += 9) {
                     const int hb = c % hbufs;
                     ptx::mbar_wait(hfull(hb), (uint32_t)((c / hbufs) & 1));
-                    if (leader && app == 0 && mi == 0) { if (c == 0) trace_mark(2); else trace_mark(2 + c); }
                     const uint32_t h_lo = (sbase + (uint32_t)(hb * halo_stride)) >> 4;
                     for (int t = (mi - kbase) & (nm - 1); t < 9; t += nm) {
                         ptx::mbar_wait(full((int)st), par);
@@ -299,7 +280,7 @@ res_tc_kernel(const __grid_constant__ CUtensorMap tma_in, const __grid_constant_
                     if (leader && !p.staged) ptx::tc_commit(hempty(hb));     // chunk done: its halo buffer may be refilled
                     __syncwarp();
                 }
-                if (leader && issuer) { ptx::tc_commit(d1full); if (app == 0 && mi == 0) trace_mark(8); }    // this issuer's GEMM1 MMAs issued
+                if (leader && issuer) ptx::tc_commit(d1full);    // this issuer's GEMM1 MMAs issued
                 if (mi == 0) {
                     // GEMM2 once the epilogue has written relu(D1) as the A2 operand
                     if (app == 0) ptx::mbar_wait(w2full, 0);
@@ -312,7 +293,7 @@ res_tc_kernel(const __grid_constant__ CUtensorMap tma_in, const __grid_constant_
                                 ptx::mma_tf32(tmem_base + d2col, ptx::smem_desc_sw128(sbase + a2_off + a * RT_A_BYTES + kk * 32),
                                               ptx::smem_desc_sw128(sbase + w2_off + a * p.C * 128 + kk * 32), idesc2,
                                               (a > 0 || kk > 0) ? 1u : 0u);
-                    if (leader) { ptx::tc_commit(d2full); if (app == 0) trace_mark(11); }   // GEMM2 issued
+                    if (leader) ptx::tc_commit(d2full);   // GEMM2 issued
                 }
                 __syncwarp();
                 if (p.staged) {
@@ -349,7 +330,6 @@ res_tc_kernel(const __grid_constant__ CUtensorMap tma_in, const __grid_constant_
         // ---- epilogue 1: relu(D1) -> A2 operand in shared memory ----
         ptx::mbar_wait_sleep(d1full, ap);
         ptx::tc_fence_after();
-        if (tid == 0 && app < 2) trace_mark(9 + 16 * app);       // GEMM1 complete (epilogue sees D1)
         for (int a = 0; a < matoms; ++a) {
             float v[32];
             if (p.nmma == 4) {                              // all four partials in flight, then one fixed-order sum
@@ -384,12 +364,10 @@ res_tc_kernel(const __grid_constant__ CUtensorMap tma_in, const __grid_constant_
         ptx::tc_fence_before();
         __syncwarp();
         if (lane == 0) ptx::mbar_arrive(a2ready);
-        if (tid == 0 && app < 2) trace_mark(10 + 16 * app);      // A2 written
 
         // ---- epilogue 2: D2 + skip -> ReLU -> next application's input / NHWC store ----
         ptx::mbar_wait_sleep(d2full, ap, 64);
         ptx::tc_fence_after();
-        if (tid == 0 && app < 2) trace_mark(12 + 16 * app);      // GEMM2 complete
         if (!last) {
             // chained application (staged mode, whole images per tile): r_{a+1} = act(r_a + D2) replaces r_a
             epilogue2_staged(0, c_split, false);
@@ -397,7 +375,6 @@ res_tc_kernel(const __grid_constant__ CUtensorMap tma_in, const __grid_constant_
             ptx::tc_fence_before();
             __syncwarp();
             if (lane == 0) ptx::mbar_arrive(actready);
-            if (tid == 0 && app == 0) trace_mark(15);            // activation rewritten in place
             continue;
         }
         if (p.staged) {
@@ -431,11 +408,9 @@ res_tc_kernel(const __grid_constant__ CUtensorMap tma_in, const __grid_constant_
         }
         }   // applications
     }
-    if (tid == 0) trace_mark(13);                    // epilogue 2 stores issued
     ptx::tc_fence_before();
     __syncthreads();
     if (warp == 5) ptx::tmem_dealloc(tmem_base, (uint32_t)tcols);
-    if (tid == 128) trace_mark(14);                      // exit
 }
 
 int rt_pow2_ceil(int x) {
@@ -461,13 +436,10 @@ int launch_res_tc(const float *r, const float *w1_tc, const float *w2_tc, float 
     if (napp > 1 && !relu_out) return VQB_ERR_UNSUPPORTED;      // a chained layer input must be relu(x)
     ResTcParams q;
     q.napp = napp;
-    {
-        static const int want = [] { const char *e = vqb_getenv("VQB_RES_NMMA"); const int v = e ? atoi(e) : 4; return (v == 1 || v == 2) ? v : 4; }();
-        q.nmma = want;
-        while (q.nmma > 1 && q.nmma * Cmid + C > 512) q.nmma >>= 1;      // TMEM columns: nmma D1 partials + D2
-        // the k-steps of every application must deal out the same way (fused == separate launches, bit for bit)
-        while (q.nmma > 1 && (9 * (C / 32)) % q.nmma != 0) q.nmma >>= 1;
-    }
+    q.nmma = 4;
+    while (q.nmma > 1 && q.nmma * Cmid + C > 512) q.nmma >>= 1;      // TMEM columns: nmma D1 partials + D2
+    // the k-steps of every application must deal out the same way (fused == separate launches, bit for bit)
+    while (q.nmma > 1 && (9 * (C / 32)) % q.nmma != 0) q.nmma >>= 1;
     q.skip = r; q.out = out; q.B = B; q.H = H; q.W = W; q.C = C; q.Cmid = Cmid; q.relu_out = relu_out;
     q.BH = rt_pow2_ceil(H) < 16 ? rt_pow2_ceil(H) : 16;
     q.BN = 16 / q.BH;
@@ -475,7 +447,7 @@ int launch_res_tc(const float *r, const float *w1_tc, const float *w2_tc, float 
     q.tiles_y = (H + q.BH - 1) / q.BH;
     const int tiles_n = (B + q.BN - 1) / q.BN;
 
-    const int RT_WP = vqb_halo_wp();
+    const int RT_WP = VQB_HALO_WP;
     q.WP = RT_WP;
     CUtensorMap tin, tw1, tw2, tout;
     // dims ordered (c, w, n, h): the BN images of a tile interleave row by row in shared memory
@@ -534,10 +506,7 @@ int launch_res_tc(const float *r, const float *w1_tc, const float *w2_tc, float 
         if (stages < RT_GROUP) return VQB_ERR_UNSUPPORTED;
     }
     q.stages = stages;
-    {
-        static const int want = [] { const char *e = vqb_getenv("VQB_RES_NPROD"); return (e && atoi(e) == 1) ? 1 : 2; }();
-        q.nprod = (q.staged && stages % 2 == 0) ? want : 1;
-    }
+    q.nprod = (q.staged && stages % 2 == 0) ? 2 : 1;
     const int smem = stages * stage_bytes + fixed;
     static int attr_max = 0;
     if (smem > attr_max) {

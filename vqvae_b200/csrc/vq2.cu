@@ -1,13 +1,15 @@
-// vq2.cu -- fused VectorQuantizer.forward on tcgen05 (sm_100a), D = 64: second-generation epilogue.
+// vq2.cu -- fused VectorQuantizer.forward on tcgen05 (sm_100a), D = 64, K <= 8192.
 //
-// Replaces quantizer.py:45-71.  Same contract and the same arithmetic argument as vq_tc.cu (round 1): the TF32
-// scores s_k = ||e_k||^2 - 2 z.e_k only SELECT; tau bounds twice the worst-case error of a score, so every code whose
-// canonical fp32 distance could be the minimum -- the winner and all its ties -- has s_k <= min_k s_k + tau; codes
-// inside that window are re-scored with the canonical chain of oracle/csrc/oracle.c (sequential fmaf over d,
-// fl(fl(A+B) - fl(2M)), first minimum wins, NaN wins), so idx / z_q are bit-identical to vq_exact.cu and the oracle.
+// Replaces quantizer.py:45-71.  Contract: idx / z_q are bit-identical to vq_exact.cu and to the oracle.  The TF32
+// scores s_k = ||e_k||^2 - 2 z.e_k only SELECT; tau bounds twice the worst-case error of a score (tf32 truncation of
+// both operands, fp32 accumulation and the rounding of the canonical formula), so every code whose canonical fp32
+// distance could be the minimum -- the winner and all its ties -- has s_k <= min_k s_k + tau; codes inside that
+// window are re-scored with the canonical chain of oracle/csrc/oracle.c (sequential fmaf over d,
+// fl(fl(A+B) - fl(2M)), first minimum wins, NaN wins).
 //
-// What changed (profiles/r01_vq_tc_epilogue_timeline.txt: 8.7 us per 128-row tile against a 1.5 us HBM budget, all
-// phases serial, every row re-scoring 8-16 codes although 82-86 % of the rows have ONE code inside the window):
+// Design (against the round-1 kernel, profiles/r01_vq_tc_epilogue_timeline.txt: 8.7 us per 128-row tile against a
+// 1.5 us HBM budget, all phases serial, every row re-scoring 8-16 codes although 82-86 % of the rows have ONE code
+// inside the window):
 //   * the sweep over the scores only takes MINIMA, over several partitions of a thread's codes at once: P1 = the
 //     column's residue mod 16 (16 running minima), P2 = its 16-column block inside the chunk pair (16 minima, reduced
 //     by a min3 tree as the block passes), and for streamed codebooks P3 / P4 = the chunk pair mod 8 / div 8.  That is
@@ -647,24 +649,69 @@ vq2_kernel(const __grid_constant__ CUtensorMap tmz, const __grid_constant__ CUte
     if (warp == 2) ptx::tmem_dealloc(tmem_base, 512);
 }
 
+// workspace prep of a streamed codebook: canonical code norms (quantizer.py:50), their maximum, a non-finite flag
+__global__ void vq2_prep_kernel(const float *__restrict__ E, int K, int Kpad, float *__restrict__ bn,
+                                unsigned *__restrict__ scal) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= Kpad) return;
+    if (k >= K) { bn[k] = __int_as_float(0x7f800000); return; }
+    const float *e = E + (size_t)k * DD;
+    float s = 0.f;
+    for (int d = 0; d < DD; ++d) s = __fadd_rn(s, __fmul_rn(e[d], e[d]));
+    bn[k] = s;
+    if (!(s < __int_as_float(0x7f800000))) atomicOr(&scal[1], 1u);       // inf or NaN
+    else atomicMax(&scal[0], __float_as_uint(sqrtf(s) * 1.00001f));       // positive floats order as uints
+}
+
+// SSE of the per-CTA partials; n < 0: the count is read from *pending (deferred reduction; 0 = sse is already final)
+__global__ void vq2_sum_partials(const double *__restrict__ partials, int n, const unsigned *__restrict__ pending,
+                                 double *__restrict__ out) {
+    __shared__ double sh[256];
+    if (n < 0) n = (int)*pending;
+    if (n <= 0) return;
+    double s = 0.0;
+    for (int i = threadIdx.x; i < n; i += 256) s += partials[i];
+    sh[threadIdx.x] = s;
+    __syncthreads();
+    for (int off = 128; off >= 1; off >>= 1) {
+        if (threadIdx.x < off) sh[threadIdx.x] += sh[threadIdx.x + off];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) *out = sh[0];
+}
+
+size_t align256(size_t x) { return (x + 255) / 256 * 256; }
+
 }  // namespace
 
 bool vq2_supported(long long N, int K, int D) {
     return D == DD && N >= 1 && N < (1LL << 31) && K >= 1 && K <= 8192;
 }
 
-size_t vq_ws_marker_offset(int K);
-size_t vq_tc_workspace_bytes(int K);
-void vq_tc_prep(const float *E, int K, int Kpad, float *bn, unsigned *scal, cudaStream_t s);
-void vq_tc_sum(const double *partials, int n, double *out, cudaStream_t s);
+// workspace: [bn: Kpad floats][scal: 256 B][partials: 256 doubles]; the deferred-reduction marker lives behind
+// both VQ kernels' workspace layouts (vq_ws_marker_offset)
+size_t vq2_workspace_bytes(int K) {
+    const size_t Kpad = (size_t)((K + CN - 1) / CN) * CN;
+    return align256(Kpad * 4) + 256 + 256 * sizeof(double);
+}
 
-// workspace layout = vq_tc.cu's: [bn: Kpad floats][scal: 256 B][partials: 256 doubles]
+size_t vq_ws_marker_offset(int K);
+
+int launch_vq_reduce_sse(const void *ws, int K, double *sse, cudaStream_t s) {
+    const int Kpad = (K + CN - 1) / CN * CN;
+    const unsigned char *w = reinterpret_cast<const unsigned char *>(ws);
+    const double *partials = reinterpret_cast<const double *>(w + align256((size_t)Kpad * 4) + 256);
+    vq2_sum_partials<<<1, 256, 0, s>>>(partials, -1, reinterpret_cast<const unsigned *>(w + vq_ws_marker_offset(K)), sse);
+    VQB_COUNT_LAUNCH(1);
+    return vqb_cuda_status(cudaGetLastError());
+}
+
+// defer != 0: the SSE partials stay in the workspace (vqb_vq_reduce_sse_f32 sums them later, e.g. on a side stream)
 int launch_vq2(const float *z, const float *E, long long N, int K, int D, long long *idx, void *zq, double *sse, int *hist,
                void *ws, int defer, int zq_bf16, cudaStream_t s) {
     if (!vq2_supported(N, K, D)) return VQB_ERR_UNSUPPORTED;
     const int nchunks = (K + CN - 1) / CN;
     const int Kpad = nchunks * CN;
-    auto align256 = [](size_t x) { return (x + 255) / 256 * 256; };
     unsigned char *w = reinterpret_cast<unsigned char *>(ws);
     float *bn = reinterpret_cast<float *>(w);
     unsigned *scal = reinterpret_cast<unsigned *>(w + align256((size_t)Kpad * 4));
@@ -682,7 +729,7 @@ int launch_vq2(const float *z, const float *E, long long N, int K, int D, long l
     if (nchunks > 2) {          // streamed codebook: norms / max / flag from a prep launch
         e = cudaMemsetAsync(scal, 0, 256, s);
         if (e != cudaSuccess) return (int)e;
-        vq_tc_prep(E, K, Kpad, bn, scal, s);
+        vq2_prep_kernel<<<(Kpad + 127) / 128, 128, 0, s>>>(E, K, Kpad, bn, scal);
         nlaunch = 3;
     }
     static bool attr_set = false;
@@ -715,7 +762,7 @@ int launch_vq2(const float *z, const float *E, long long N, int K, int D, long l
                       : vqb_launch(vq2_kernel<false, false>, gd, bd, (size_t)SMEM_ALLOC, s, tmz, tme, p);
     if (le != cudaSuccess)
         return (int)le;
-    if (!defer) vq_tc_sum(partials, grid, sse, s);
+    if (!defer) vq2_sum_partials<<<1, 256, 0, s>>>(partials, grid, nullptr, sse);
     VQB_COUNT_LAUNCH(defer ? nlaunch - 1 : nlaunch);
     return vqb_cuda_status(cudaGetLastError());
 }

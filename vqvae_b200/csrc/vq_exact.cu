@@ -13,7 +13,8 @@
 //     torch.argmin), merged across the 16 threads of a row with shuffles;
 //   * the same launch gathers e_idx, writes z_q = z + (e - z), accumulates the SSE and a
 //     shared-memory code histogram that is flushed once per CTA.
-// This is the bit-exact kernel and the checker for the tcgen05 kernel in vq_tc.cu.
+// This is the bit-exact kernel, the checker for the tcgen05 kernel in vq2.cu and the kernel for every shape vq2 does
+// not cover (D != 64 or K > 8192).
 #include "common.cuh"
 
 namespace {

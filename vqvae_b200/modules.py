@@ -513,13 +513,15 @@ class VQVAE(nn.Module):
 
     def _bf16_pipeline(self):
         """True when set_precision("bf16") is active AND every layer of this model has a bf16 tcgen05 kernel
-        (h_dim = 128 family: 64-channel first layer, channel counts in multiples of 64, embedding_dim = 64).
+        (h_dim = 128 family: 64-channel first layer, channel counts in multiples of 64, embedding_dim = 64,
+        n_embeddings <= 8192 for the VQ kernel that writes bf16 z_q).
         Other shapes run the TF32 kernels on fp32 activations, with a one-time warning."""
         if get_precision() != "bf16":
             return False
         pq = self.pre_quantization_conv
+        vq = self.vector_quantization
         ok = (self.encoder._bf16_ok() and self.decoder._bf16_ok() and pq.in_channels % 64 == 0
-              and pq.out_channels == 64 and self.vector_quantization.e_dim == 64)
+              and pq.out_channels == 64 and vq.e_dim == 64 and vq.n_e <= 8192)
         if not ok and not getattr(self, "_warned_bf16", False):
             import warnings
             warnings.warn("vqvae_b200: this model shape has no bf16 kernels; precision 'bf16' runs the TF32 kernels")

@@ -360,28 +360,9 @@ def relu_(x):
     return x
 
 
-VQ_KERNELS = {"auto": 0, "exact": 1, "tc": 2, "tc_r1": 3}
+VQ_KERNELS = {"auto": 0, "exact": 1, "tc": 2}
 
 
 def set_vq_kernel(name: str):
-    """Kernel used by vq_forward: "auto" (tcgen05 when D == 64), "exact" (FFMA) or "tc"."""
+    """Kernel used by vq_forward: "auto" (tcgen05 when D == 64 and K <= 8192), "exact" (FFMA) or "tc"."""
     check(lib().vqb_set_vq_kernel(VQ_KERNELS[name]), "set_vq_kernel")
-
-
-def vq_debug_scores(z_rows, codebook):
-    """Diagnostic: tcgen05 VQ kernel + dump of its approximate TF32 scores (N, Kpad)."""
-    N, D = z_rows.shape
-    K = codebook.shape[0]
-    dev = z_rows.device
-    kpad = (K + 255) // 256 * 256
-    idx = torch.empty((N,), dtype=torch.int64, device=dev)
-    zq = torch.empty((N, D), dtype=torch.float32, device=dev)
-    sse = torch.empty((1,), dtype=torch.float64, device=dev)
-    hist = torch.empty((K,), dtype=torch.int32, device=dev)
-    scores = torch.full((N, kpad), float("nan"), dtype=torch.float32, device=dev)
-    ws_bytes = lib().vqb_vq_workspace_bytes(N, K, D)
-    ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
-    check(lib().vqb_debug_vq_scores_f32(z_rows.data_ptr(), codebook.data_ptr(), N, K, D, idx.data_ptr(),
-                                        zq.data_ptr(), sse.data_ptr(), hist.data_ptr(), ws.data_ptr(),
-                                        ws_bytes, scores.data_ptr(), _stream()), "vq_debug_scores")
-    return idx, zq, sse, hist, scores
